@@ -12,6 +12,8 @@ Lipschitz RGB MLP, 256^3 occupancy grid of the analytic sphere SDF |x|-0.3. A st
 importance resampling, forward, losses, backward through the double backward, dense AdamW.
   python bench.py --rays 8192 ...                          same step with more rays per GPU (BASELINE config 4 = 8192 rays/GPU x 8 GPUs)
   python bench.py --workload sphere_trace [--gpus N]       sphere-traced render of one 1920x1080 frame (BASELINE config 5): px/s
+  python bench.py ... --dump-outputs DIR                   training workload: after the timed steps, write what the last one computed
+                                                           as DIR/<name>.npy
 
 Metric: rays/s (whole job). `value`: inputs resident on the device. `e2e`: per step the ray indices come from pinned
 host memory and the loss is read back. Multi-GPU: rays sharded by rank (weak scaling), one NCCL all-reduce of the
@@ -200,6 +202,7 @@ def run_ours(args):
         # peer: fused gradient reduction + AdamW + parameter broadcast over NVLink peer memory (no all-reduce); nccl: one all-reduce
         # captured in the optimizer graph; nccl_overlap: bucketed all-reduce overlapped with the SDF backward / AdamW
         tr.enable_data_parallel(world, overlap=(dp_mode == "nccl_overlap"), mode="peer" if dp_mode == "peer" else "nccl")
+    start = StartState(tr) if args.dump_outputs else None      # before the first step (the peer mode above re-homes the buffers)
 
     def one_step(i, e2e):
         # e2e: the step's inputs start in pinned host memory; otherwise they are device resident
@@ -226,6 +229,7 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     static_eager = False
+    last = {}
 
     def timed(e2e, with_events, steps=None):
         steps = args.steps if steps is None else steps
@@ -239,9 +243,11 @@ def run_ours(args):
         nsamples = 0
         with ClockSampler(local) as cs:
             for i in range(args.warmup, args.warmup + steps):
+                if start is not None and e2e and i == args.warmup + steps - 1:
+                    start.restore()             # the last timed step: its inputs are the same in every run
                 s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 s.record()
-                one_step(i, e2e)
+                last["loss"] = one_step(i, e2e)
                 e.record()
                 evs.append((s, e))
                 if not graphed:
@@ -258,6 +264,8 @@ def run_ours(args):
 
     ms_dev, launches, ktimes, clocks, avg_samples = timed(e2e=False, with_events=not graphed)
     ms_e2e, _, _, clocks2, _ = timed(e2e=True, with_events=False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, training_outputs(tr, last["loss"]))
     ms_per_step = ms_dev / args.steps
     prof_steps = 0
     if graphed:
@@ -461,6 +469,64 @@ def run_sphere_trace(args):
         dist.destroy_process_group()
 
 
+DUMP_SAMPLE = 1 << 20          # entries kept of each large state buffer by --dump-outputs
+DUMP_LIMIT = 64 << 20
+
+
+class StartState:
+    """The model state a Trainer is built with (parameters, AdamW moments, occupancy grid), put back in place before the last timed
+    step when outputs are dumped. Every training step accumulates gradients, losses and grid updates with floating-point atomics in
+    an order that changes from run to run, and AdamW (eps 1e-15) and the curvature loss magnify those last-bit differences: after 25
+    steps of this workload the losses of two runs differed by up to 15 % (B200, 1000 W). Restored, the last step reads the same
+    parameters, grid and rays in every run, so its outputs differ only by the rounding of that one step."""
+
+    def __init__(self, tr):
+        opt, grid = tr.optimizer, tr.occupancy_grid
+        if not hasattr(opt, "flat_param"):
+            raise RuntimeError("--dump-outputs needs the flat-buffer optimizer (not --modular)")
+        self.tr = tr
+        self.live = [opt.flat_param, opt.exp_avg, opt.exp_avg_sq, grid.get_grid_values(), grid.get_grid_occupancy()]
+        self.saved = [t.clone() for t in self.live]
+
+    def restore(self):
+        for dst, src in zip(self.live, self.saved):
+            dst.copy_(src)
+        fused = getattr(self.tr.model_sdf, "fused", None)
+        if fused is not None:
+            fused.repack()                      # the fused SDF kernels read a packed copy of the MLP weights
+        torch.cuda.synchronize()                # graphs on other streams read these buffers too
+
+
+def training_outputs(tr, loss):
+    """What a training step leaves its caller: the loss and its terms, the sample count, and the parameters and AdamW moments the
+    optimizer step wrote (a fixed seeded sample of DUMP_SAMPLE entries of each: the flat buffers hold ~17M floats apiece)."""
+    out = {"loss": np.array([float(loss)], np.float64)}
+    for k in ("loss_rgb", "loss_eikonal", "loss_curvature", "nr_samples_dev"):
+        if torch.is_tensor(tr.last.get(k)):
+            out[k] = tr.last[k].detach().double().cpu().numpy().reshape(-1)
+    opt = tr.optimizer
+    if hasattr(opt, "flat_param"):
+        bufs = {"params": opt.flat_param, "adam_exp_avg": opt.exp_avg, "adam_exp_avg_sq": opt.exp_avg_sq}
+    else:
+        bufs = {"params": torch.cat([p.detach().reshape(-1) for p in tr.params])}
+    for name, b in bufs.items():
+        n = b.numel()
+        idx = np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_SAMPLE), replace=False))
+        out[name + "_sample"] = b.detach().reshape(-1)[torch.from_numpy(idx).to(b.device)].float().cpu().numpy()
+    return out
+
+
+def dump_outputs(d, arrays):
+    """DIR/<name>.npy per array (float32 / float64), at most DUMP_LIMIT bytes in all"""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 NCU_KERNEL_OF = {"psdf_sdf_fused_forward": "k_sdf_fused_dual", "psdf_sdf_fused_backward": "k_sdf_fused_backward",
                  "psdf_sdf_fused_forward_multi": "k_sdf_fused_dual", "psdf_sdf_fused_backward_multi": "k_sdf_fused_backward",
                  "psdf_rgb_fused_forward": "k_rgb_fused", "psdf_rgb_fused_backward": "k_rgb_fused_backward",
@@ -531,7 +597,12 @@ def main():
     ap.add_argument("--width", type=int, default=1920)
     ap.add_argument("--height", type=int, default=1080)
     ap.add_argument("--trace_iters", type=int, default=256)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "train" or args.impl != "ours"):
+        # the sphere-trace frame is rendered from a 400-step SDF fit that accumulates with atomics like training (see StartState): two
+        # runs gave frames differing in ~5 % of the pixel values (B200, 1000 W)
+        ap.error("--dump-outputs covers the training workload of our implementation")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,17 +1,20 @@
 """GPU parity tests of the ray-path kernels (through the C ABI / the `permuto_sdf` mirror) against
  (a) the C oracle (oracle/rayops_oracle.c) and
- (b) the reference's own CUDA kernels compiled for sm_100a (oracle/_ref/libpsdf_ref_gpu.so) when present.
+ (b) the reference's own CUDA kernels compiled for sm_100a (oracle/_ref/libpsdf_ref_gpu.so) where built, their stored outputs
+     elsewhere (tests/ref_golden.py).
 Integer / index results must match bit for bit; float results within the tolerance written in each test
 (north star: <= 1e-3 relative; we hold the ray path to <= 1e-6 absolute and report bit-exact fractions)."""
 import numpy as np
 import pytest
 import torch
 
+import ref_golden
 import scenes
 from oracle import rayops as orc
 from oracle import ref_gpu
 
 pytestmark = pytest.mark.gpu
+_fresh_generators = pytest.fixture(autouse=True)(ref_golden.fresh_generators)
 
 V = 128
 FTOL = 2e-6
@@ -53,10 +56,9 @@ def test_sphere_ray_intersection(scene):
     assert np.array_equal(N(got[4]), exp[4])
     for g, e, name in zip(got[:4], exp[:4], ["pts_entry", "t_entry", "pts_exit", "t_exit"]):
         assert np.array_equal(N(g), e), name + " not bit-exact vs oracle"
-    if ref_gpu.available():
-        ref = ref_gpu.sphere_ray_intersection(scenes.SPHERE_RADIUS, [0, 0, 0], T(o), T(d))
-        for g, e, name in zip(got, ref, ["pts_entry", "t_entry", "pts_exit", "t_exit", "hit"]):
-            assert torch.equal(g, e), name + " not bit-exact vs reference kernel"
+    ref = ref_golden.once(lambda: ref_gpu.sphere_ray_intersection(scenes.SPHERE_RADIUS, [0, 0, 0], T(o), T(d)))
+    for i, (g, name) in enumerate(zip(got, ["pts_entry", "t_entry", "pts_exit", "t_exit", "hit"])):
+        ref_golden.equal("rayops.sphere." + name, g, lambda i=i: ref()[i])
 
 
 def test_sphere_points(scene):
@@ -69,8 +71,7 @@ def test_sphere_points(scene):
     out = torch.empty(1000, 3, device="cuda")
     call("psdf_sphere_rand_points_inside", 1000, 0.5, phi, ct, u, out)
     close(N(out), orc.sphere_rand_points_inside(0.5, N(phi), N(ct), N(u)), 1e-6, "rand_points_inside")
-    if ref_gpu.available():
-        close(N(out), N(ref_gpu.sphere_rand_points_inside(0.5, [0, 0, 0], phi, ct, u)), 1e-6, "rand_points_inside vs ref")
+    ref_golden.close("rayops.rand_points_inside", out, lambda: ref_gpu.sphere_rand_points_inside(0.5, [0, 0, 0], phi, ct, u), 1e-6)
 
 
 # --------------------------------------------------------------------------------------------------- Occupancy grid
@@ -82,16 +83,14 @@ def test_grid_points(scene, randomize):
     pts = g.compute_grid_points(randomize)
     exp = orc.occ_grid_points(V, 1.0, [0, 0, 0], None, randomize, st, inc)
     assert np.array_equal(N(pts), exp)
-    if ref_gpu.available():
-        assert torch.equal(pts, ref_gpu.occ_grid_points(V, 1.0, [0, 0, 0], None, randomize, st, inc))
+    ref_golden.equal("rayops.grid_points.r%d" % randomize, pts, lambda: ref_gpu.occ_grid_points(V, 1.0, [0, 0, 0], None, randomize, st, inc))
     torch.manual_seed(5)
     st = OccupancyGrid.m_rng.state
     p2, idx = g.compute_random_sample_of_grid_points(5000, randomize)
     assert idx.dtype == torch.int32 and int(idx.max()) < V ** 3
     exp2 = orc.occ_grid_points(V, 1.0, [0, 0, 0], N(idx), randomize, st, inc)
     assert np.array_equal(N(p2), exp2)
-    if ref_gpu.available():
-        assert torch.equal(p2, ref_gpu.occ_grid_points(V, 1.0, [0, 0, 0], idx, randomize, st, inc))
+    ref_golden.equal("rayops.grid_points_subset.r%d" % randomize, p2, lambda: ref_gpu.occ_grid_points(V, 1.0, [0, 0, 0], idx, randomize, st, inc))
 
 
 def test_grid_updates_and_lookup(scene):
@@ -103,10 +102,11 @@ def test_grid_updates_and_lookup(scene):
     g.update_with_sdf(sdf, 512.0, 1e10, 1e-4)
     assert np.array_equal(N(g.get_grid_occupancy()).astype(np.uint8), scene["occ"]), "occupancy bits differ from oracle"
     assert np.array_equal(N(g.get_grid_values()), scene["values"])
-    if ref_gpu.available():
+    def ref_occupancy():
         rv, ro = torch.ones(V ** 3, device="cuda"), torch.ones(V ** 3, dtype=torch.bool, device="cuda")
         ref_gpu.occ_update_with_sdf(V, 1.0, sdf, None, 512.0, 1e-4, rv, ro)
-        assert torch.equal(ro, g.get_grid_occupancy()), "occupancy bits differ from the reference kernel"
+        return ro
+    ref_golden.equal("rayops.update_with_sdf.occupancy", g.get_grid_occupancy(), ref_occupancy)
     # random-sample sdf update (1.0 half diagonals, inv_s from a tensor)
     idx = torch.from_numpy(rng.permutation(V ** 3)[:20000].astype(np.int32)).cuda()
     s2 = torch.from_numpy(rng.uniform(-0.05, 0.05, (20000, 1)).astype(np.float32)).cuda()
@@ -130,8 +130,7 @@ def test_grid_updates_and_lookup(scene):
     q = torch.from_numpy(rng.uniform(-0.7, 0.7, (50000, 3)).astype(np.float32)).cuda()
     got = scene["grid"].check_occupancy(q)
     assert np.array_equal(N(got), orc.occ_check_occupancy(V, 1.0, [0, 0, 0], scene["occ"], N(q)))
-    if ref_gpu.available():
-        assert torch.equal(got, ref_gpu.occ_check_occupancy(V, 1.0, [0, 0, 0], scene["grid"].get_grid_occupancy(), q))
+    ref_golden.equal("rayops.check_occupancy", got, lambda: ref_gpu.occ_check_occupancy(V, 1.0, [0, 0, 0], scene["grid"].get_grid_occupancy(), q))
 
 
 def per_ray(pk_start_end, arrs):
@@ -170,17 +169,14 @@ def test_samples_in_occupied_regions(scene, jitter):
         assert np.array_equal(N(a), b)
     idx = comp.compute_per_sample_ray_idx(comp.ray_start_end_idx, comp.samples_pos.shape[0])
     assert np.array_equal(N(idx), orc.packed_per_sample_ray_idx(ecomp.start_end, ecomp.cur))
-    if ref_gpu.available():
-        ref = ref_gpu.occ_samples_in_occupied_regions(V, 1.0, [0, 0, 0], T(o), T(d), te, tx, scene["grid"].get_grid_occupancy(), 1e-3, 64,
-                                                      jitter, st, inc)
-        rse = N(ref.start_end)
-        assert np.array_equal(rse[:, 1] - rse[:, 0], se[:, 1] - se[:, 0]), "per-ray sample counts differ from the reference kernel"
-        assert torch.equal(ref.fixed_dt, rsp.ray_fixed_dt)
-        rz, rdt, rpos = N(ref.z), N(ref.dt), N(ref.pos)
-        gz, gdt, gpos = N(rsp.samples_z), N(rsp.samples_dt), N(rsp.samples_pos)
-        for (s, e), (rs, re) in zip(se, rse):
-            assert np.array_equal(gz[s:e], rz[rs:re]) and np.array_equal(gdt[s:e], rdt[rs:re]) and np.array_equal(gpos[s:e], rpos[rs:re]), \
-                "samples not bit exact vs the reference kernel"
+    ref = ref_golden.once(lambda: ref_gpu.occ_samples_in_occupied_regions(V, 1.0, [0, 0, 0], T(o), T(d), te, tx, scene["grid"].get_grid_occupancy(),
+                                                                         1e-3, 64, jitter, st, inc))
+    key = "rayops.occ_samples.j%d." % jitter
+    ref_golden.equal(key + "counts", ref_golden.counts(se), lambda: ref_golden.counts(ref().start_end))
+    ref_golden.equal(key + "fixed_dt", rsp.ray_fixed_dt, lambda: ref().fixed_dt)
+    ours = ref_golden.per_ray(se, rsp.samples_z, rsp.samples_dt, rsp.samples_pos)
+    for i, name in enumerate(("z", "dt", "pos")):
+        ref_golden.equal(key + name, ours[i], lambda i=i: ref_golden.per_ray(ref().start_end, ref().z, ref().dt, ref().pos)[i])
 
 
 def test_first_sample_and_advance(scene):
@@ -192,24 +188,22 @@ def test_first_sample_and_advance(scene):
     assert np.array_equal(se, exp.start_end)
     for (s, e) in se:
         assert np.array_equal(N(rsp.samples_pos)[s:e], exp.pos[s:e]) and np.array_equal(N(rsp.samples_z)[s:e], exp.z[s:e])
-    if ref_gpu.available():
-        ref = ref_gpu.occ_first_sample_start(V, 1.0, [0, 0, 0], T(o), T(d), te, tx, scene["grid"].get_grid_occupancy())
-        rse = N(ref.start_end)
-        assert np.array_equal(rse[:, 1] - rse[:, 0], se[:, 1] - se[:, 0])
-        for (s, e), (rs, re) in zip(se, rse):
-            assert np.array_equal(N(rsp.samples_pos)[s:e], N(ref.pos)[rs:re])
+    ref = ref_golden.once(lambda: ref_gpu.occ_first_sample_start(V, 1.0, [0, 0, 0], T(o), T(d), te, tx, scene["grid"].get_grid_occupancy()))
+    ref_golden.equal("rayops.first_sample.counts", ref_golden.counts(se), lambda: ref_golden.counts(ref().start_end))
+    ref_golden.equal("rayops.first_sample.pos", ref_golden.per_ray(se, rsp.samples_pos)[0], lambda: ref_golden.per_ray(ref().start_end, ref().pos)[0])
     comp = rsp.compact_to_valid_samples()
     pos = comp.samples_pos + comp.samples_dirs * (0.5 / V)
     # move some points into empty space (towards the centre of the object, which is unoccupied inside)
     pos = (pos * 0.2).contiguous()
     expect_pos, expect_within = orc.occ_advance_to_next_occupied(V, 1.0, [0, 0, 0], N(comp.samples_dirs), N(pos), scene["occ"])
-    if ref_gpu.available():
-        rpos, rwithin = ref_gpu.occ_advance_to_next_occupied(V, 1.0, [0, 0, 0], comp.samples_dirs, pos, scene["grid"].get_grid_occupancy())
+    pos_in = pos.clone()                                # ours moves pos in place
+    ref = ref_golden.once(lambda: ref_gpu.occ_advance_to_next_occupied(V, 1.0, [0, 0, 0], comp.samples_dirs, pos_in,
+                                                                      scene["grid"].get_grid_occupancy()))
     newpos, within = scene["grid"].advance_sample_to_next_occupied_voxel(comp.samples_dirs, pos)
     assert newpos.data_ptr() == pos.data_ptr(), "output must alias the input like the reference"
     assert np.array_equal(N(within), expect_within) and np.array_equal(N(newpos), expect_pos)
-    if ref_gpu.available():
-        assert torch.equal(within, rwithin) and torch.equal(newpos, rpos)
+    ref_golden.equal("rayops.advance.within", within, lambda: ref()[1])
+    ref_golden.equal("rayops.advance.pos", newpos, lambda: ref()[0])
 
 
 # --------------------------------------------------------------------------------------------------- RaySampler
@@ -226,12 +220,9 @@ def test_sampler_fg_bg(scene, jitter):
     for (s, e) in se:
         assert np.array_equal(N(fg.samples_z)[s:e], exp.z[s:e]) and np.array_equal(N(fg.samples_pos)[s:e], exp.pos[s:e])
         assert np.array_equal(N(fg.samples_dt)[s:e], exp.dt[s:e])
-    if ref_gpu.available():
-        ref = ref_gpu.sampler_fg(T(o), T(d), te, tx, 0.5, [0, 0, 0], 0.01, 48, jitter, st, inc)
-        rse = N(ref.start_end)
-        assert np.array_equal(rse[:, 1] - rse[:, 0], se[:, 1] - se[:, 0])
-        for (s, e), (rs, re) in zip(se, rse):
-            assert np.array_equal(N(fg.samples_z)[s:e], N(ref.z)[rs:re])
+    ref = ref_golden.once(lambda: ref_gpu.sampler_fg(T(o), T(d), te, tx, 0.5, [0, 0, 0], 0.01, 48, jitter, st, inc))
+    ref_golden.equal("rayops.sampler_fg.j%d.counts" % jitter, ref_golden.counts(se), lambda: ref_golden.counts(ref().start_end))
+    ref_golden.equal("rayops.sampler_fg.j%d.z" % jitter, ref_golden.per_ray(se, fg.samples_z)[0], lambda: ref_golden.per_ray(ref().start_end, ref().z)[0])
     st, inc = RaySampler.m_rng.state, RaySampler.m_rng.inc
     bg = RaySampler.compute_samples_bg(T(o), T(d), tx, 32, 0.5, [0.0, 0.0, 0.0], jitter, False)
     eb = orc.sampler_bg(o, d, N(tx), 32, 0.5, [0, 0, 0], jitter, False, st, inc)
@@ -242,11 +233,11 @@ def test_sampler_fg_bg(scene, jitter):
     close(N(bg.samples_z)[sel], eb.z[sel], 1e-3, "bg z")        # z = t_exit / t can be ~1e3: relative 1e-6
     assert np.allclose(N(bg.samples_z)[sel], eb.z[sel], rtol=2e-6, atol=1e-6)
     assert np.allclose(N(bg.samples_pos_4d)[sel], eb.pos4[sel], rtol=2e-5, atol=2e-6)
-    if ref_gpu.available():
-        rb = ref_gpu.sampler_bg(T(o), T(d), tx, 32, 0.5, [0, 0, 0], jitter, False, st, inc)
-        assert np.allclose(N(bg.samples_z)[sel], N(rb.z)[sel], rtol=2e-6, atol=1e-6)
-        assert np.allclose(N(bg.samples_pos_4d)[sel], N(rb.pos4)[sel], rtol=2e-5, atol=2e-6)
-        assert np.allclose(N(bg.samples_dt)[sel], N(rb.dt)[sel], rtol=1e-4, atol=1e-5)
+    rb = ref_golden.once(lambda: ref_gpu.sampler_bg(T(o), T(d), tx, 32, 0.5, [0, 0, 0], jitter, False, st, inc))
+    key = "rayops.sampler_bg.j%d." % jitter
+    ref_golden.close(key + "z", N(bg.samples_z)[sel], lambda: N(rb().z)[sel], 1e-6, 2e-6)
+    ref_golden.close(key + "pos4", N(bg.samples_pos_4d)[sel], lambda: N(rb().pos4)[sel], 2e-6, 2e-5)
+    ref_golden.close(key + "dt", N(bg.samples_dt)[sel], lambda: N(rb().dt)[sel], 1e-5, 1e-4)
 
 
 # --------------------------------------------------------------------------------------------------- statics
@@ -259,8 +250,7 @@ def test_spherical_harmonics(cuda, degree):
     got = PermutoSDF.spherical_harmonics(T(d), degree)
     assert got.shape == (3001, degree * degree)
     close(N(got), orc.spherical_harmonics(d, degree), 2e-6, "SH vs oracle")
-    if ref_gpu.available():
-        close(N(got), N(ref_gpu.spherical_harmonics(T(d), degree)), 2e-6, "SH vs reference kernel")
+    ref_golden.close("rayops.sh.deg%d" % degree, got, lambda: ref_gpu.spherical_harmonics(T(d), degree), 2e-6)
 
 
 def test_random_rays_from_reel(cuda):
@@ -280,6 +270,7 @@ def test_random_rays_from_reel(cuda):
     assert torch.equal(img, img2)
     eo, ed, egt, egm = orc.random_rays_from_reel(rgb, mask, K, tf, N(pix), N(img))
     close(N(o), eo, 0, "origins"); close(N(d), ed, 1e-6, "dirs"); close(N(gt), egt, 0, "gt rgb"); close(N(gm), egm, 0, "mask")
-    if ref_gpu.available():
-        ro, rd, rgt, rgm = ref_gpu.random_rays_from_reel(T(rgb), T(mask), T(K), T(tf), pix, img)
-        close(N(d), N(rd), 1e-6, "dirs vs ref"); assert torch.equal(gt, rgt) and torch.equal(gm, rgm) and torch.equal(o, ro)
+    ref = ref_golden.once(lambda: ref_gpu.random_rays_from_reel(T(rgb), T(mask), T(K), T(tf), pix, img))
+    ref_golden.close("rayops.reel.dirs", d, lambda: ref()[1], 1e-6)
+    for i, (g, name) in enumerate(((o, "origins"), (gt, "gt"), (gm, "mask"))):
+        ref_golden.equal("rayops.reel." + name, g, lambda i=i: ref()[(0, 2, 3)[i]])

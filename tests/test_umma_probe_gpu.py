@@ -20,7 +20,7 @@ def _probe(mode, A, A2, B):
     return dump.cpu()
 
 
-def test_two_m64_accumulators_interleave_by_lane_offset_16():
+def test_two_m64_accumulators_interleave_by_lane_offset_16(cuda):
     torch.manual_seed(0)
     A, A2, B = (torch.randn(128, 64, device="cuda") for _ in range(3))
     dump = _probe(0, A, A2, B)
@@ -34,7 +34,7 @@ def test_two_m64_accumulators_interleave_by_lane_offset_16():
     assert e0 < 1e-4 and e1 < 1e-4
 
 
-def test_reverse_gemm_from_forward_weight_tile_mn_major_b():
+def test_reverse_gemm_from_forward_weight_tile_mn_major_b(cuda):
     torch.manual_seed(1)
     A, A2, W = (torch.randn(128, 64, device="cuda") for _ in range(3))
     dump = _probe(1, A, A2, W)

@@ -1,15 +1,17 @@
-"""GPU parity tests of the volume-compositing / importance-resampling kernels against the C oracle and,
-when present, the reference's own CUDA kernels (oracle/_ref). Tolerances are written per test; the
-serial-order recurrences are expected to be bit exact."""
+"""GPU parity tests of the volume-compositing / importance-resampling kernels against the C oracle and the
+reference's own CUDA kernels (oracle/_ref where built, their stored outputs elsewhere: tests/ref_golden.py).
+Tolerances are written per test; the serial-order recurrences are expected to be bit exact."""
 import numpy as np
 import pytest
 import torch
 
+import ref_golden
 import scenes
 from oracle import rayops as orc
 from oracle import ref_gpu
 
 pytestmark = pytest.mark.gpu
+_fresh_generators = pytest.fixture(autouse=True)(ref_golden.fresh_generators)
 V = 128
 
 
@@ -72,7 +74,7 @@ def test_scans_and_sums(packed):
     rsp = packed["rsp"]
     Ns, R = rsp.samples_z.shape[0], rsp.ray_start_end_idx.shape[0]
     p = to_oracle(rsp)
-    rp = to_ref(rsp) if ref_gpu.available() else None
+    rp = ref_golden.once(lambda: to_ref(rsp))
     g = torch.Generator(device="cuda").manual_seed(0)
     alpha = torch.rand(Ns, 1, device="cuda", generator=g) * 0.2 + 0.8
     Tt, bg = VR.cumprod_alpha2transmittance(rsp, alpha)
@@ -86,26 +88,24 @@ def test_scans_and_sums(packed):
         sr, ss = VR.sum_over_each_ray(rsp, v)
         er, es = orc.vr_sum(p, N(v))
         eq(N(sr), er, "sum ray D=%d" % D); eq(N(ss), es, "sum sample D=%d" % D)
-        if rp is not None:
-            rr, rs = ref_gpu.vr_sum(rp, v)
-            eq(N(sr), N(rr), "sum ray vs ref D=%d" % D); eq(N(ss), N(rs), "sum sample vs ref")
+        ref = ref_golden.once(lambda: ref_gpu.vr_sum(rp(), v))
+        ref_golden.equal("volrender.sum_ray.D%d" % D, sr, lambda: ref()[0])
+        ref_golden.equal("volrender.sum_sample.D%d" % D, ss, lambda: ref()[1])
         if D <= 3:
             gr, gs = torch.rand(R, D, device="cuda", generator=g), torch.rand(Ns, D, device="cuda", generator=g)
             gb = VR.sum_over_each_ray_backward(gr, gs, rsp, v)
             eq(N(gb), orc.vr_sum_backward(p, N(gr), N(gs)), "sum backward")
-            if rp is not None:
-                eq(N(gb), N(ref_gpu.vr_sum_backward(rp, gr, gs, v)), "sum backward vs ref")
+            ref_golden.equal("volrender.sum_backward.D%d" % D, gb, lambda: ref_gpu.vr_sum_backward(rp(), gr, gs, v))
     for inv in (False, True):
         eq(N(VR.cumsum_over_each_ray(rsp, w, inv)), orc.vr_cumsum(p, N(w), inv), "cumsum inverse=%s" % inv)
     eq(N(VR.compute_cdf(rsp, w)), orc.vr_cdf(p, N(w)), "cdf")
     eq(N(VR.compute_dt(rsp, packed["tx"], True)), orc.vr_compute_dt(p, N(packed["tx"]), True), "compute_dt")
-    if rp is not None:
-        rT, rbg = ref_gpu.vr_cumprod(rp, alpha)
-        eq(N(Tt), N(rT), "T vs ref"); eq(N(bg), N(rbg), "bg vs ref")
-        eq(N(VR.integrate_with_weights(rsp, rgb, w)), N(ref_gpu.vr_integrate(rp, rgb, w)), "integrate vs ref")
-        eq(N(VR.cumsum_over_each_ray(rsp, w, True)), N(ref_gpu.vr_cumsum(rp, w, True)), "rev cumsum vs ref")
-        eq(N(VR.compute_cdf(rsp, w)), N(ref_gpu.vr_cdf(rp, w)), "cdf vs ref")
-        eq(N(VR.compute_dt(rsp, packed["tx"], False)), N(ref_gpu.vr_compute_dt(rp, packed["tx"], False)), "dt vs ref")
+    ref = ref_golden.once(lambda: ref_gpu.vr_cumprod(rp(), alpha))
+    ref_golden.equal("volrender.T", Tt, lambda: ref()[0]); ref_golden.equal("volrender.bg", bg, lambda: ref()[1])
+    ref_golden.equal("volrender.integrate", VR.integrate_with_weights(rsp, rgb, w), lambda: ref_gpu.vr_integrate(rp(), rgb, w))
+    ref_golden.equal("volrender.rev_cumsum", VR.cumsum_over_each_ray(rsp, w, True), lambda: ref_gpu.vr_cumsum(rp(), w, True))
+    ref_golden.equal("volrender.cdf", VR.compute_cdf(rsp, w), lambda: ref_gpu.vr_cdf(rp(), w))
+    ref_golden.equal("volrender.dt", VR.compute_dt(rsp, packed["tx"], False), lambda: ref_gpu.vr_compute_dt(rp(), packed["tx"], False))
     # backward kernels
     gT = torch.rand(Ns, 1, device="cuda", generator=g)
     gbg = torch.rand(R, 1, device="cuda", generator=g)
@@ -122,10 +122,10 @@ def test_scans_and_sums(packed):
     gv2, gw2 = VR.integrate_with_weights_backward(gp, rsp, rgb, w, pred)
     VR.reference_bugs = False
     eq(N(gw2), orc.vr_integrate_backward(p, N(gp), N(rgb), N(w), True)[1], "integrate backward weights (reference bug mode)")
-    if rp is not None:
-        eq(N(ga), N(ref_gpu.vr_cumprod_backward(rp, gT, gbg, alpha, Tt, bg, cs)), "cumprod backward vs ref", 1e-6)
-        rv, rw = ref_gpu.vr_integrate_backward(rp, gp, rgb, w, pred)
-        eq(N(gv2), N(rv), "integrate backward vals vs ref"); eq(N(gw2), N(rw), "integrate backward weights vs ref (bug mode)")
+    ref_golden.close("volrender.cumprod_backward", ga, lambda: ref_gpu.vr_cumprod_backward(rp(), gT, gbg, alpha, Tt, bg, cs), 1e-6)
+    ref = ref_golden.once(lambda: ref_gpu.vr_integrate_backward(rp(), gp, rgb, w, pred))
+    ref_golden.equal("volrender.integrate_backward.vals", gv2, lambda: ref()[0])
+    ref_golden.equal("volrender.integrate_backward.weights_bug_mode", gw2, lambda: ref()[1])
 
 
 def test_nerf_render(packed):
@@ -144,13 +144,12 @@ def test_nerf_render(packed):
     grgb, grad = VR.volume_render_nerf_backward(gp, gb, torch.zeros(Ns, 1, device="cuda"), pr, rsp, rgb, rad, packed["tx"], False, bg)
     e1, e2 = orc.vr_render_nerf_backward(p, N(gp), N(gb), N(pr), N(bg), N(rgb), N(rad))
     eq(N(grgb), e1, "nerf g_rgb", 2e-5); eq(N(grad), e2, "nerf g_radiance", 2e-4)
-    if ref_gpu.available():
-        rp = to_ref(rsp)
-        rr = ref_gpu.vr_render_nerf(rp, packed["tx"], rgb, rad)
-        for a, b, n in zip((pr, dp, bg, w), rr, ("rgb", "depth", "bg", "w")):
-            eq(N(a), N(b), "nerf vs ref " + n, 1e-6)
-        r1, r2 = ref_gpu.vr_render_nerf_backward(rp, gp, gb, pr, packed["tx"], bg, rgb, rad)
-        eq(N(grgb), N(r1), "nerf g_rgb vs ref", 1e-6); eq(N(grad), N(r2), "nerf g_radiance vs ref", 1e-5)
+    rr = ref_golden.once(lambda: ref_gpu.vr_render_nerf(to_ref(rsp), packed["tx"], rgb, rad))
+    for i, (a, n) in enumerate(zip((pr, dp, bg, w), ("rgb", "depth", "bg", "w"))):
+        ref_golden.close("volrender.nerf." + n, a, lambda i=i: rr()[i], 1e-6)
+    rb = ref_golden.once(lambda: ref_gpu.vr_render_nerf_backward(to_ref(rsp), gp, gb, pr, packed["tx"], bg, rgb, rad))
+    ref_golden.close("volrender.nerf.g_rgb", grgb, lambda: rb()[0], 1e-6)
+    ref_golden.close("volrender.nerf.g_radiance", grad, lambda: rb()[1], 1e-5)
 
 
 @pytest.mark.parametrize("jitter", [False, True])
@@ -165,8 +164,8 @@ def test_importance_resampling(packed, jitter):
     p = to_oracle(rsp)
     alpha = VR.sdf2alpha(rsp, sdf, 512, True, 1.0)
     eq(N(alpha), orc.vr_sdf2alpha(p, N(sdf), 512, True, 1.0), "sdf2alpha", 5e-6)   # expf ulp
-    if ref_gpu.available():
-        eq(N(alpha), N(ref_gpu.vr_sdf2alpha(to_ref(rsp), sdf, 512, True, 1.0)), "sdf2alpha vs ref", 2e-6)
+    key = "volrender.importance.j%d." % jitter
+    ref_golden.close(key + "sdf2alpha", alpha, lambda: ref_gpu.vr_sdf2alpha(to_ref(rsp), sdf, 512, True, 1.0), 2e-6)
     alpha = alpha.clip(0.0, 1.0)
     Tt, _ = VR.cumprod_alpha2transmittance(rsp, 1 - alpha + 1e-7)
     w = alpha * Tt
@@ -178,9 +177,9 @@ def test_importance_resampling(packed, jitter):
     eimp = orc.vr_importance_sample(N(o), N(d), p, N(cdf), 16, jitter, st, inc)
     assert imp.rays_have_equal_nr_of_samples and imp.fixed_nr_of_samples_per_ray == 16
     eq(N(imp.samples_z), eimp.z, "importance z"); eq(N(imp.samples_pos), eimp.pos, "importance pos")
-    if ref_gpu.available():
-        rimp = ref_gpu.vr_importance_sample(o, d, to_ref(rsp), cdf, 16, jitter, st, inc)
-        eq(N(imp.samples_z), N(rimp.z), "importance z vs ref"); eq(N(imp.samples_pos), N(rimp.pos), "importance pos vs ref")
+    rimp = ref_golden.once(lambda: ref_gpu.vr_importance_sample(o, d, to_ref(rsp), cdf, 16, jitter, st, inc))
+    ref_golden.equal(key + "z", imp.samples_z, lambda: rimp().z)
+    ref_golden.equal(key + "pos", imp.samples_pos, lambda: rimp().pos)
     sdf_imp = (imp.samples_pos.norm(dim=1, keepdim=True) - scenes.OBJECT_RADIUS).contiguous()
     imp.set_sdf(sdf_imp)
     eimp.sdf, eimp.has_sdf = N(sdf_imp), True
@@ -199,14 +198,16 @@ def test_importance_resampling(packed, jitter):
         assert np.all(np.diff(zz[s:e, 0]) >= 0), "merged samples must be sorted by z"
     cc = comb.compact_to_valid_samples()
     assert cc.samples_pos.shape[0] == n and cc.has_sdf
-    if ref_gpu.available():
-        rimp.sdf, rimp.has_sdf = sdf_imp, True
-        rcomb = ref_gpu.vr_combine(o, d, tx, to_ref(rsp), rimp)
-        rse = N(rcomb.start_end)
-        assert np.array_equal(rse[:, 1] - rse[:, 0], se[:, 1] - se[:, 0])
-        for (s, e), (rs, re) in zip(se, rse):
-            for a, b in [(comb.samples_z, rcomb.z), (comb.samples_dt, rcomb.dt), (comb.samples_pos, rcomb.pos), (comb.samples_sdf, rcomb.sdf)]:
-                assert np.array_equal(N(a)[s:e], N(b)[rs:re]), "merged samples differ from the reference kernel"
+    def ref_combine():
+        r = rimp()
+        r.sdf, r.has_sdf = sdf_imp, True
+        return ref_gpu.vr_combine(o, d, tx, to_ref(rsp), r)
+    rcomb = ref_golden.once(ref_combine)
+    ref_golden.equal(key + "combined.counts", ref_golden.counts(se), lambda: ref_golden.counts(rcomb().start_end))
+    ours = ref_golden.per_ray(se, comb.samples_z, comb.samples_dt, comb.samples_pos, comb.samples_sdf)
+    for i, nm in enumerate(("z", "dt", "pos", "sdf")):
+        ref_golden.equal(key + "combined." + nm, ours[i],
+                         lambda i=i: ref_golden.per_ray(rcomb().start_end, rcomb().z, rcomb().dt, rcomb().pos, rcomb().sdf)[i])
     rsp.remove_sdf()
 
 
